@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W            # this framework, one rank per GPU
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU reference arm (oracle port)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also write the last timed step's outputs
+
+With --dump-outputs the inputs, the seeds and the number of steps before the dumped one are fixed by the arguments,
+so two builds of the project can be compared output for output (dump_outputs lists what is written).
 
 Workload (BASELINE.json configs[1]): models/train_rels.py step of MotifNet SGCls — VGG16 backbone
 (frozen), batch 6 x 3 x 592 x 592 synthetic images per GPU, 20 GT boxes and 15 GT relations per image
@@ -45,6 +49,8 @@ def parse():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0; see dump_outputs)")
     return ap.parse_args()
 
 
@@ -101,12 +107,14 @@ class ClockSampler(object):
 
 # ------------------------------------------------------------------------------------------ model setup
 def build_model(device, seed=0):
+    import numpy as np
     import torch
     from lib.rel_model import RelModel
     from dataloaders.synthetic import synthetic_model_state
     classes = ['__background__'] + ['obj%d' % i for i in range(150)]
     rels = ['__background__'] + ['rel%d' % i for i in range(50)]
     torch.manual_seed(seed)
+    np.random.seed(seed)        # the relation / RoI sampling draws from numpy's global RNG
     # scripts/train_models_sgcls.sh:19-21
     m = RelModel(classes, rels, mode='sgcls', num_gpus=1, require_overlap_det=True, use_resnet=False, order='leftright',
                  nl_edge=4, nl_obj=2, hidden_dim=512, use_proposals=False, pass_in_obj_feats_to_decoder=False,
@@ -133,9 +141,10 @@ def get_optim(model, lr):
     return FlatSGD([(fc, lr / 10.0), (non_fc, lr)], momentum=0.9, weight_decay=1e-4, max_norm=5.0, defer_step=True)
 
 
-def train_step(model, optimizer, reducer=None, fwd_tuple=None, blob=None):
+def train_step(model, optimizer, reducer=None, fwd_tuple=None, blob=None, keep=None):
     """models/train_rels.py:118-152 (train_batch): forward, two cross-entropies, backward, clip 5, step.
-    The data-parallel gradient average is one all-reduce per flat gradient buffer."""
+    The data-parallel gradient average is one all-reduce per flat gradient buffer.
+    `keep` (a dict), when given, receives the step's Result and loss tensor."""
     from torch.nn import functional as F
     import torch.distributed as dist
     result = model[blob] if blob is not None else model(*fwd_tuple)
@@ -152,7 +161,44 @@ def train_step(model, optimizer, reducer=None, fwd_tuple=None, blob=None):
     loss.backward()
     optimizer.all_reduce_grads()
     optimizer.step()
+    if keep is not None:
+        keep["result"], keep["loss"] = result, loss.detach()
     return float(loss.detach())  # the reference's train_batch reads the losses back every step (train_rels.py:151)
+
+
+DUMP_MAX_ELEMS = 1 << 18        # per array: 1 MB as float32, 2 MB as float64 (< 64 MB over all Result fields)
+PARAM_SAMPLE = 1 << 14
+
+
+def dump_outputs(out_dir, model, last):
+    """--dump-outputs: what a caller of the timed step receives from its last step, one DIR/<name>.npy each:
+    `loss`, every tensor field of the training Result (`rm_obj_dists`, `rel_dists`, `rel_labels`, ...) and
+    `trainable_params` (the parameters the step's update left, PARAM_SAMPLE seeded elements of each trainable
+    parameter in named_parameters() order, all of a smaller one). An array larger than DUMP_MAX_ELEMS elements is
+    written as `<name>_sample`, a seeded sample of its flattened elements. Floating arrays are float32, integer ones
+    float64 (exact)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+
+    def sample(flat, k, seed):
+        idx = np.random.RandomState(seed).randint(0, flat.numel(), k)
+        return flat[torch.from_numpy(idx).to(flat.device)]
+
+    arrays = {"loss": last["loss"].reshape(1)}
+    for name, v in vars(last["result"]).items():
+        if not torch.is_tensor(v):
+            continue
+        v = v.detach()
+        if v.numel() > DUMP_MAX_ELEMS:
+            name, v = name + "_sample", sample(v.reshape(-1), DUMP_MAX_ELEMS, 0)
+        arrays[name] = v
+    params = [p.detach().reshape(-1) for _, p in model.named_parameters() if p.requires_grad]
+    arrays["trainable_params"] = torch.cat([p if p.numel() <= PARAM_SAMPLE else sample(p, PARAM_SAMPLE, i)
+                                            for i, p in enumerate(params)])
+    for name, v in arrays.items():
+        v = v.cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (v.float() if v.is_floating_point() else v.double()).numpy())
 
 
 def settle_warmup(step, sync, world, dev, min_steps=12, max_steps=60, tol=1.03):
@@ -249,8 +295,10 @@ def run_b200(args):
         train_step(model, opt, reducer, fwd_tuple=resident[i % len(resident)])
     # A fresh box keeps paging libraries in and autotuning for a while: keep warming up (untimed) until
     # the step time has settled — at least 12 extra steps and the last five within 3 % of each other and of the best — or 60 extra steps.
+    # With --dump-outputs every run takes the longest warm-up, so that the dumped step starts from the same parameters,
+    # optimizer state and RNG state whatever the timings were.
     extra = settle_warmup(lambda i: train_step(model, opt, reducer, fwd_tuple=resident[i % len(resident)]),
-                          torch.cuda.synchronize, world, dev)
+                          torch.cuda.synchronize, world, dev, min_steps=60 if args.dump_outputs else 12)
     W += extra
     # Python's cyclic GC pauses the host for tens of ms when a generation-2 pass lands in a step (seen as one
     # 90 ms step among 21.7 ms ones): collect now, freeze what survived, and keep the collector off inside the
@@ -273,9 +321,14 @@ def run_b200(args):
     W += 2
     mem0 = torch.cuda.memory_stats(dev)
     calls0 = motifs_cabi.LAUNCHER_CALLS
-    ms_res = timed(lambda i: train_step(model, opt, reducer, fwd_tuple=resident[i % len(resident)]), args.steps)
+    last = {} if args.dump_outputs and rank == 0 else None
+    ms_res = timed(lambda i: train_step(model, opt, reducer, fwd_tuple=resident[i % len(resident)],
+                                        keep=last if i == args.steps - 1 else None), args.steps)
     calls = motifs_cabi.LAUNCHER_CALLS - calls0
     steps_res = list(timed.last_per_step)
+    if last is not None:
+        dump_outputs(args.dump_outputs, model, last)
+        last.clear()
     # e2e: public API with host buffers; H2D of the batch and D2H of the loss every step
     losses = []
 

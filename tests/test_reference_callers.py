@@ -1,22 +1,17 @@
-"""The reference's CALLER code executed against the product's API surface (SURVEY.md section 8b "Model API").
-
-`models/train_rels.py` (get_optim :57-72, train_batch :118-152) and `models/eval_rels.py` (val_batch :59-86) are parsed from
-/root/reference with `ast`, their function definitions are extracted UNEDITED apart from the documented compat shim
-below, and are executed here against
+"""The caller code of `models/train_rels.py` (get_optim :57-72, train_batch :118-152) and `models/eval_rels.py` (val_batch
+:59-86) against the product's API surface (SURVEY.md section 8b "Model API"):
   * the product's `RelModel` class — `detector[b]` (`__getitem__` + `Blob.scatter` protocol), `detector.train()/eval()`,
     `named_parameters()` with the `roi_fmap*` prefixes, the training `Result` fields and the eval 5-tuple,
   * the product's `lib.pytorch_misc.clip_grad_norm`, `lib.evaluation.sg_eval.BasicSceneGraphEvaluator`, `config` constants,
   * `dataloaders.synthetic.SyntheticBlob` standing in for `dataloaders/blob.py:Blob`.
-The one thing that is NOT the product here is the arithmetic of `forward`: the product has no CPU path (by design) and
-/root/reference does not exist on the GPU box, so the two can never meet in one process. `forward` is therefore delegated
-to the oracle restatement operating ON THE PRODUCT'S OWN Parameter objects (the oracle modules are re-pointed at them), so
-that the callers' `loss.backward()`, `clip_grad_norm(detector.named_parameters())` and `optimizer.step()` act on the
-product model. The same step with the product's kernels is held to the oracle on the GPU (tests/test_model_gpu.py, and
-tests/test_callers_gpu.py runs the restated caller sequence end to end there).
-
-Compat shim (INTEGRATION.md section 3): `x.data[0]` (PyTorch-0.3 indexing of a 0-dim tensor) -> `float(x)`; the `verbose=`
-keyword of ReduceLROnPlateau (removed from torch) is dropped. Nothing else is rewritten."""
-import ast
+The caller sequence is restated here in this repository's words and held to tests/golden/reference_callers.npz: what the
+reference's OWN function definitions computed when tests/golden/make_golden_callers.py executed them, unedited apart
+from a small compat shim, against the same product surface and inputs. Neither needs the reference tree at test time.
+The one thing that is NOT the product here is the arithmetic of `forward`: the product has no CPU path (by design).
+`forward` is therefore delegated to the oracle restatement operating ON THE PRODUCT'S OWN Parameter objects (the oracle
+modules are re-pointed at them), so that the callers' `loss.backward()`, `clip_grad_norm(detector.named_parameters())` and
+`optimizer.step()` act on the product model. The same step with the product's kernels is held to the oracle on the GPU
+(tests/test_model_gpu.py, and tests/test_callers_gpu.py runs the restated caller sequence end to end there)."""
 import os
 import sys
 import types
@@ -25,35 +20,9 @@ import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_callers.npz")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree is only present in the build container")
-
-
-class _Shim(ast.NodeTransformer):
-    def visit_Subscript(self, node):
-        self.generic_visit(node)
-        if isinstance(node.value, ast.Attribute) and node.value.attr == "data" and \
-                isinstance(node.slice, ast.Constant) and node.slice.value == 0:
-            return ast.copy_location(ast.Call(func=ast.Name(id="float", ctx=ast.Load()), args=[node.value.value], keywords=[]), node)
-        return node
-
-    def visit_Call(self, node):
-        self.generic_visit(node)
-        if isinstance(node.func, ast.Name) and node.func.id == "ReduceLROnPlateau":
-            node.keywords = [k for k in node.keywords if k.arg != "verbose"]
-        return node
-
-
-def _function(path, name, namespace):
-    """exec the (shimmed) definition of top-level function `name` of the reference file into `namespace`."""
-    tree = ast.parse(open(path).read())
-    node = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == name)
-    mod = ast.fix_missing_locations(_Shim().visit(ast.Module(body=[node], type_ignores=[])))
-    exec(compile(mod, path, "exec"), namespace)
-    return namespace[name]
 
 
 _BUILT = {}
@@ -114,37 +83,89 @@ def _ones_masks(orc, n_obj, n_rel, n_img):
     orc.detector.masks, orc.masks, orc.context.masks = ones(det), ones(top), ones(ctx)
 
 
-def test_train_rels_get_optim_and_train_batch_run_against_the_product():
-    import pandas as pd
-    from torch import optim
-    from torch.nn import functional as F
-    from torch.optim.lr_scheduler import ReduceLROnPlateau
-    from lib.pytorch_misc import clip_grad_norm
-    from dataloaders.synthetic import make_numpy_batch, SyntheticBlob
+TRAIN_CONF = dict(adam=False, l2=1e-4, lr=6e-3, clip=5.0, mode="sgcls", num_gpus=1, print_interval=100)
+PARAM_SAMPLE = 64
+
+
+def train_case():
+    """The product surface with its detector frozen (train_rels.py:51-52), the run's config and one synthetic batch."""
+    from dataloaders.synthetic import make_numpy_batch
     detector, orc, state = _build("sgcls")
-    for n, param in detector.detector.named_parameters():            # train_rels.py:51-52
+    for n, param in detector.detector.named_parameters():
         param.requires_grad = False
-    conf = types.SimpleNamespace(adam=False, l2=1e-4, lr=6e-3, clip=5.0, mode="sgcls", num_gpus=1, print_interval=100)
-    ns = dict(detector=detector, conf=conf, optim=optim, ReduceLROnPlateau=ReduceLROnPlateau, F=F, pd=pd,
-              clip_grad_norm=clip_grad_norm)
-    path = os.path.join(REF, "models", "train_rels.py")
-    optimizer, scheduler = _function(path, "get_optim", ns)(conf.lr)
-    assert [g["lr"] for g in optimizer.param_groups] == [conf.lr / 10.0, conf.lr]
-    assert len(optimizer.param_groups[0]["params"]) == 8              # fc6 / fc7 weights + biases of roi_fmap and roi_fmap_obj
-    ns["optimizer"] = optimizer
-    train_batch = _function(path, "train_batch", ns)
     B, boxes = 1, 6
     nb = make_numpy_batch(B, seed=5, boxes_per_img=boxes, rels_per_img=5)
     _ones_masks(orc, B * boxes, B * boxes * (boxes - 1), B)
     orc.detector.rng = np.random.RandomState(7)
+    return detector, orc, state, types.SimpleNamespace(**TRAIN_CONF), nb
+
+
+def eval_case():
+    """The product surface in eval mode, one synthetic image and the `val` dataset fields val_batch reads."""
+    from config import BOX_SCALE, IM_SCALE
+    from dataloaders.synthetic import make_numpy_batch
+    detector, orc, _ = _build("sgcls")
+    detector.eval()
+    nb = make_numpy_batch(1, seed=9, boxes_per_img=7, rels_per_img=6)
+    val = types.SimpleNamespace(gt_classes=[nb["gt_classes"][:, 1].copy()],
+                                relationships=[nb["gt_rels"][:, 1:].copy()],
+                                gt_boxes=[nb["gt_boxes"] * BOX_SCALE / IM_SCALE])
+    return detector, nb, val, types.SimpleNamespace(mode="sgcls", num_gpus=1)
+
+
+def param_samples(model):
+    """PARAM_SAMPLE seeded elements of every parameter (all of a smaller one), in named_parameters() order."""
+    out = []
+    for i, (_, p) in enumerate(model.named_parameters()):
+        flat = p.detach().reshape(-1)
+        if flat.numel() > PARAM_SAMPLE:
+            flat = flat[torch.from_numpy(np.random.RandomState(i).randint(0, flat.numel(), PARAM_SAMPLE))]
+        out.append(flat)
+    return torch.cat(out).numpy()
+
+
+def test_train_rels_get_optim_and_train_batch_run_against_the_product():
+    import pandas as pd
+    from torch.nn import functional as F
+    from torch.optim.lr_scheduler import ReduceLROnPlateau
+    from lib.pytorch_misc import clip_grad_norm
+    from dataloaders.synthetic import SyntheticBlob
+    gold = np.load(GOLDEN)
+    detector, orc, state, conf, nb = train_case()
+    B, boxes = 1, 6
+    # get_optim: SGD with momentum and L2, the roi_fmap* fc layers at a tenth of the rate; plateau schedule
+    named = [(n, p) for n, p in detector.named_parameters() if p.requires_grad]
+    optimizer = torch.optim.SGD([{"params": [p for n, p in named if n.startswith("roi_fmap")], "lr": conf.lr / 10.0},
+                                 {"params": [p for n, p in named if not n.startswith("roi_fmap")]}],
+                                lr=conf.lr, momentum=0.9, weight_decay=conf.l2)
+    scheduler = ReduceLROnPlateau(optimizer, "max", patience=3, factor=0.1, threshold=0.0001, threshold_mode="abs",
+                                  cooldown=1)
+    assert [g["lr"] for g in optimizer.param_groups] == [conf.lr / 10.0, conf.lr] == gold["train_lrs"].tolist()
+    assert len(optimizer.param_groups[0]["params"]) == 8              # fc6 / fc7 weights + biases of roi_fmap and roi_fmap_obj
     before = {n: p.detach().clone() for n, p in detector.named_parameters()}
     detector.train()
-    res = train_batch(SyntheticBlob(nb, "cpu"), verbose=False)
+    # train_batch: detector[b]; object + relation cross-entropies; backward; global-norm clip; step; losses as a Series
+    result = detector[SyntheticBlob(nb, "cpu")]
+    losses = {"class_loss": F.cross_entropy(result.rm_obj_dists, result.rm_obj_labels),
+              "rel_loss": F.cross_entropy(result.rel_dists, result.rel_labels[:, -1])}
+    total = losses["class_loss"] + losses["rel_loss"]
+    optimizer.zero_grad()
+    total.backward()
+    clip_grad_norm([(n, p) for n, p in detector.named_parameters() if p.grad is not None], max_norm=conf.clip, clip=True)
+    optimizer.step()
+    losses["total"] = total
+    res = pd.Series({k: float(v) for k, v in losses.items()})
     assert set(res.index) == {"class_loss", "rel_loss", "total"} and abs(res["total"] - res["class_loss"] - res["rel_loss"]) < 1e-5
     moved = [n for n, p in detector.named_parameters() if not torch.equal(p, before[n])]
     assert moved and all(not n.startswith("detector.") for n in moved)       # the frozen detector did not move
     assert any(n.startswith("roi_fmap_obj.") for n in moved) and any(n.startswith("context.obj_ctx_rnn") for n in moved)
     scheduler.step(0.1); scheduler.step(0.1)                                 # the recipe's plateau schedule accepts it
+
+    # what the reference's own get_optim / train_batch did to the same product surface
+    for k in res.index:
+        assert abs(res[k] - float(gold["train_" + k])) < 1e-5 * max(1.0, abs(res[k])), k
+    assert moved == gold["train_moved"].tolist()
+    np.testing.assert_allclose(param_samples(detector), gold["train_params"], rtol=1e-5, atol=1e-7)
 
     # the same step taken by an independent oracle model with torch's own clip + SGD gives the same loss and update
     from oracle import model as OM
@@ -170,26 +191,30 @@ def test_train_rels_get_optim_and_train_batch_run_against_the_product():
         assert torch.allclose(p, want[n], rtol=1e-5, atol=1e-7), n
 
 
+
 def test_eval_rels_val_batch_runs_against_the_product():
     from config import BOX_SCALE, IM_SCALE
     from lib.evaluation.sg_eval import BasicSceneGraphEvaluator
-    from dataloaders.synthetic import make_numpy_batch, SyntheticBlob
-    detector, orc, _ = _build("sgcls")
-    detector.eval()
-    nb = make_numpy_batch(1, seed=9, boxes_per_img=7, rels_per_img=6)
-    val = types.SimpleNamespace(gt_classes=[nb["gt_classes"][:, 1].copy()],
-                                relationships=[nb["gt_rels"][:, 1:].copy()],
-                                gt_boxes=[nb["gt_boxes"] * BOX_SCALE / IM_SCALE])
-    conf = types.SimpleNamespace(mode="sgcls", num_gpus=1)
-    all_pred_entries = []
-    ns = dict(detector=detector, conf=conf, val=val, np=np, BOX_SCALE=BOX_SCALE, IM_SCALE=IM_SCALE,
-              all_pred_entries=all_pred_entries)
-    val_batch = _function(os.path.join(REF, "models", "eval_rels.py"), "val_batch", ns)
+    from dataloaders.synthetic import SyntheticBlob
+    gold = np.load(GOLDEN)
+    detector, nb, val, conf = eval_case()
     evaluator = BasicSceneGraphEvaluator.all_modes()
+    # val_batch: one (boxes, classes, scores, rel pairs, rel scores) tuple per image with num_gpus == 1
     with torch.no_grad():
-        val_batch(0, SyntheticBlob(nb, "cpu"), evaluator)
-    assert len(all_pred_entries) == 1
-    e = all_pred_entries[0]
+        boxes_i, objs_i, obj_scores_i, rels_i, pred_scores_i = detector[SyntheticBlob(nb, "cpu")]
+    assert np.all(objs_i[rels_i[:, 0]] > 0) and np.all(objs_i[rels_i[:, 1]] > 0)
+    gt_entry = {"gt_classes": val.gt_classes[0].copy(), "gt_relations": val.relationships[0].copy(),
+                "gt_boxes": val.gt_boxes[0].copy()}
+    e = {"pred_boxes": boxes_i * BOX_SCALE / IM_SCALE, "pred_classes": objs_i, "pred_rel_inds": rels_i,
+         "obj_scores": obj_scores_i, "rel_scores": pred_scores_i}
+    evaluator[conf.mode].evaluate_scene_graph_entry(gt_entry, e)
     assert e["pred_boxes"].shape == (7, 4) and e["pred_rel_inds"].shape == (42, 2) and e["rel_scores"].shape == (42, 51)
     rec = evaluator["sgcls"].result_dict["sgcls_recall"]
     assert all(len(rec[k]) == 1 and 0.0 <= rec[k][0] <= 1.0 for k in (20, 50, 100))
+
+    # what the reference's own val_batch recorded and scored on the same product surface
+    for k in ("pred_classes", "pred_rel_inds"):
+        assert np.array_equal(e[k], gold["eval_" + k]), k
+    for k in ("pred_boxes", "obj_scores", "rel_scores"):
+        np.testing.assert_allclose(e[k], gold["eval_" + k], rtol=1e-5, atol=1e-7, err_msg=k)
+    assert [rec[k][0] for k in (20, 50, 100)] == gold["eval_recall"].tolist()
